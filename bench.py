@@ -2,6 +2,7 @@
 """bench.py -- queries/sec of one training step of the hot path (BASELINE.json configs).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cuda] [--config a|b|c|d|e]
+                    [--dump-outputs DIR]
 
 A "step" = scorer forward + fused loss/gradient + scorer backward + gradient all-reduce (N>1) + optimizer step over one
 batch of synthetic MSLR-shaped queries per GPU (weak scaling).  Default --config b = BASELINE.json configs[1], the
@@ -281,6 +282,31 @@ def algorithmic(cfg, B):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def scorer_state(ranker):
+    """name -> tensor of the scorer's checkpoint (what ranker.save writes): the weights the step updated."""
+    if hasattr(ranker, "point_sf"):
+        return dict(ranker.point_sf.state_dict())
+    return {f"{part}.{k}": v for part, m in ranker.list_sf.items() for k, v in m.state_dict().items()}
+
+
+def dump_outputs(out_dir, loss, state):
+    """DIR/loss.npy and DIR/state.<name>.npy (float32) of one train step, so that two builds can be compared output for
+    output.  Past DUMP_LIMIT_BYTES in all, each tensor is cut to a fixed, seeded sample of its flattened elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    arrays.update((f"state.{k}", v.detach().float().cpu().numpy()) for k, v in state.items())
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, a.size * DUMP_LIMIT_BYTES // total)
+            idx = np.sort(np.random.default_rng(SEED).choice(a.size, size=keep, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_b200(args, cfg):
     import torch.distributed as dist
     from ptranking_b200 import _lib, LABEL_TYPE
@@ -333,6 +359,8 @@ def run_b200(args, cfg):
     launches = _lib.launch_count() - l0
     value = world * B * args.steps / (ms / 1e3)
     last_loss = float(loss)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, scorer_state(ranker))
 
     # ---- strong scaling: the N=1 global batch split over the ranks ----------------
     strong = None
@@ -510,7 +538,8 @@ def build_roofline(cfg, B, tm, steps_timed, ms_per_step):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 100 for configs a, b, e; 20 for c; 50 for d)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "reference-cuda"])
     ap.add_argument("--config", default="b", choices=["a", "b", "c", "d", "e"], help="BASELINE.json configs[0..4]")
@@ -519,11 +548,15 @@ def main():
     ap.add_argument("--docs", type=int, default=256, help="config e: documents per query (32..1024)")
     ap.add_argument("--enc-layers", type=int, default=6, help="config c: encoder layers (6 = code default, 3 = test JSON)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss, updated scorer state) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     cfg = make_config(args)
-    if args.config != "b" and args.steps == 100:
-        args.steps = {"a": 100, "c": 20, "d": 50, "e": 100}[args.config]
+    if args.steps is None:
+        args.steps = {"a": 100, "b": 100, "c": 20, "d": 50, "e": 100}[args.config]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args, cfg, "cpu")
     elif args.impl == "reference-cuda":

@@ -1,12 +1,17 @@
 """Generate the golden fixtures in this directory by running the UNMODIFIED reference.
 
-Run in the authoring container only (the GPU box has no /root/reference):
+Run where the reference checkout is importable (the tests themselves never need it):
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PTRANKING_REFERENCE=<reference checkout> PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
 
-Imports wildltr/ptranking from /root/reference, feeds it seeded synthetic inputs
+Imports wildltr/ptranking from $PTRANKING_REFERENCE, feeds it seeded synthetic inputs
 (seed 137 = ptranking/ltr_global.py:5) and stores inputs + outputs as .npz.
 Nothing from the reference is copied: only tensors it computed are saved.
+
+scorers.npz / train_steps.npz keep each file small: features and the pointwise scorers' initial weights are not
+stored -- tests/helpers.py::load regenerates them from the same seeds and checks them against the stored
+``<key>@probe`` elements -- and the pointwise scorers' gradients above 1024 elements are stored as a strided sample
+plus their L2 norm and sum (put_sampled; tests/helpers.py::sampled reproduces the sampling).
 """
 import os
 import sys
@@ -20,7 +25,9 @@ REF = os.environ.get("PTRANKING_REFERENCE", "/root/reference")
 sys.path.insert(0, REF)
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
 
+from helpers import probe, sampled, synth_labels  # noqa: E402
 from ptranking.data.data_utils import LABEL_TYPE  # noqa: E402
 from ptranking.ltr_adhoc.pairwise.ranknet import RankNet  # noqa: E402
 from ptranking.ltr_adhoc.listwise.lambdarank import LambdaRank  # noqa: E402
@@ -38,14 +45,18 @@ MQ_P = np.array([12279, 2001, 931], dtype=np.float64)
 MQ_P /= MQ_P.sum()
 
 
-def synth_labels(rng, B, n, probs, presort=True):
-    y = rng.choice(len(probs), size=(B, n), p=probs).astype(np.float32)
-    for b in range(B):
-        if y[b].max() < 1:
-            y[b, rng.integers(n)] = float(rng.integers(1, len(probs)))
-    if presort:
-        y = -np.sort(-y, axis=1)
-    return y
+def put_sampled(out, key, arr):
+    """``arr`` in full when small, else its strided sample plus the whole tensor's L2 norm and sum."""
+    arr = np.asarray(arr)
+    s = sampled(arr)
+    out[key] = arr.copy() if s.size == arr.size else s
+    if s.size < arr.size:
+        out[key + "@norm"] = np.float64(np.sqrt((arr.astype(np.float64) ** 2).sum()))
+        out[key + "@sum"] = np.float64(arr.astype(np.float64).sum())
+
+
+def put_probe(out, key, arr):
+    out[key + "@probe"] = probe(arr)
 
 
 def point_sf_dict(F, **over):
@@ -222,11 +233,12 @@ def scorer_fixtures():
             s = r.forward(X)
             (s * rvec).sum().backward()
             key = f"point_{name}_B{B}_n{n}_F{F}"
-            out[key + "__X"] = X.numpy(); out[key + "__dscores"] = rvec.numpy()
+            put_probe(out, key + "__X", X.numpy()); out[key + "__dscores"] = rvec.numpy()
             out[key + "__scores"] = s.detach().numpy()
-            _flatten_sd(key + "__param", r.point_sf.state_dict(), out)
+            for k, v in r.point_sf.state_dict().items():
+                put_probe(out, f"{key}__param::{k}", v.numpy())
             for k, p in r.point_sf.named_parameters():
-                out[f"{key}__grad::{k}"] = p.grad.numpy().copy()
+                put_sampled(out, f"{key}__grad::{k}", p.grad.numpy())
     for enc in ("DASALC", "AllRank", "AttnDIN"):
         for bn in (False, True):
             torch.manual_seed(137)
@@ -273,14 +285,15 @@ def train_fixtures():
             for part in ("head_ffnns", "encoder", "tail_ffnns"):
                 _flatten_sd(f"{name}__init::{part}", r.list_sf[part].state_dict(), out)
         else:
-            _flatten_sd(f"{name}__init", r.point_sf.state_dict(), out)
+            for k, v in r.point_sf.state_dict().items():
+                put_probe(out, f"{name}__init::{k}", v.numpy())
         X = rng.standard_normal((3, B, n, F)).astype(np.float32)
         y = np.stack([synth_labels(rng, B, n, MSLR_P) for _ in range(3)])
         losses = []
         for t in range(3):
             loss, _ = r.train_op(torch.from_numpy(X[t]), torch.from_numpy(y[t]), presort=True, label_type=ML)
             losses.append(float(loss.detach()))
-        out[name + "__X"] = X; out[name + "__labels"] = y
+        put_probe(out, name + "__X", X); out[name + "__labels"] = y
         out[name + "__losses"] = np.array(losses, dtype=np.float64)
         if is_list:
             for part in ("head_ffnns", "encoder", "tail_ffnns"):

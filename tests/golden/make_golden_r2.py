@@ -8,9 +8,11 @@
 
     PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden_r2.py      ->  scorers_r2.npz
 
-To keep the file small, tensors above 16384 elements are stored as a strided sample (every k-th element of the flattened
-tensor) plus their L2 norm and sum -- tests/helpers.py::sampled() reproduces the sampling; the initial weights are stored
-in full (make_clones gives every encoder layer the same initial weights, list_ranker.py:48-50, so one layer is stored).
+To keep the file small, outputs above 1024 elements are stored as a strided sample (every k-th element of the flattened
+tensor) plus their L2 norm and sum -- tests/helpers.py::sampled() reproduces the sampling.  Features and initial
+weights are not stored: tests/helpers.py::load regenerates them from the same seeds and checks them against the stored
+``<key>@probe`` elements (make_clones gives every encoder layer the same initial weights, list_ranker.py:48-50, so one
+layer is probed).
 """
 import os
 import sys
@@ -27,17 +29,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.dirname(HERE))
 
-from make_golden import synth_labels, point_sf_dict, MSLR_P, ML, _flatten_sd  # noqa: E402
-from helpers import sampled  # noqa: E402
+from make_golden import synth_labels, point_sf_dict, MSLR_P, ML, put_probe, put_sampled  # noqa: E402
 from ptranking.ltr_adhoc.listwise.listnet import ListNet  # noqa: E402
 from ptranking.ltr_adhoc.listwise.approxNDCG import ApproxNDCG  # noqa: E402
-
-
-def put_sampled(out, key, arr):
-    arr = np.asarray(arr)
-    out[key] = sampled(arr)
-    out[key + "@norm"] = np.float64(np.sqrt((arr.astype(np.float64) ** 2).sum()))
-    out[key + "@sum"] = np.float64(arr.astype(np.float64).sum())
 
 
 def main():
@@ -59,10 +53,12 @@ def main():
             s = r.forward(X)
             (s * rvec).sum().backward()
             key = f"point_af{code}_B{B}_n{n}_F{F}"
-            out[key + "__X"], out[key + "__dscores"], out[key + "__scores"] = X.numpy(), rvec.numpy(), s.detach().numpy()
-            _flatten_sd(key + "__param", r.point_sf.state_dict(), out)
+            put_probe(out, key + "__X", X.numpy())
+            out[key + "__dscores"], out[key + "__scores"] = rvec.numpy(), s.detach().numpy()
+            for k, v in r.point_sf.state_dict().items():
+                put_probe(out, f"{key}__param::{k}", v.numpy())
             for k, p in r.point_sf.named_parameters():
-                out[f"{key}__grad::{k}"] = p.grad.numpy().copy()
+                put_sampled(out, f"{key}__grad::{k}", p.grad.numpy())
 
     # ---- list scorer at config (c)'s real shape ----------------------------------------------------
     B, n, F = 2, 512, 136
@@ -76,17 +72,20 @@ def main():
         r.eval_mode()           # the tail FFN ignores the configured dropout (SURVEY B10): eval mode switches it off
         key = f"listc_{tag}"
         out[key + "__L"] = np.int64(L)
-        _flatten_sd(f"{key}__init::head_ffnns", r.list_sf["head_ffnns"].state_dict(), out)
-        _flatten_sd(f"{key}__init::tail_ffnns", r.list_sf["tail_ffnns"].state_dict(), out)
+        for part in ("head_ffnns", "tail_ffnns"):
+            for k, v in r.list_sf[part].state_dict().items():
+                put_probe(out, f"{key}__init::{part}::{k}", v.numpy())
         enc_sd = r.list_sf["encoder"].state_dict()
         layer0 = {k[len("layers.0."):]: v for k, v in enc_sd.items() if k.startswith("layers.0.")}
         for l in range(1, L):   # make_clones: identical initial weights in every layer
             for k, v in layer0.items():
                 assert torch.equal(enc_sd[f"layers.{l}.{k}"], v)
-        _flatten_sd(f"{key}__init::encoder_layer", layer0, out)
+        for k, v in layer0.items():
+            put_probe(out, f"{key}__init::encoder_layer::{k}", v.numpy())
         X = rng.standard_normal((3, B, n, F)).astype(np.float32)
         y = np.stack([synth_labels(rng, B, n, MSLR_P) for _ in range(3)])
-        out[key + "__X"], out[key + "__labels"] = X, y
+        put_probe(out, key + "__X", X)
+        out[key + "__labels"] = y
         # forward + every parameter gradient for a random upstream gradient
         rvec = torch.from_numpy(rng.standard_normal((B, n)).astype(np.float32))
         s = r.forward(torch.from_numpy(X[0]))

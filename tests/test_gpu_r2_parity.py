@@ -6,8 +6,7 @@ import pytest
 import torch
 
 from oracle import ref_port as rp
-from tests.helpers import load, rel_err, sampled
-from tests.test_oracle_vs_golden import point_cfg
+from tests.helpers import load, point_cfg, reference_point_outputs, rel_err, sampled
 from tests.test_oracle_r2 import AF_CODES, LISTC
 from tests.test_gpu_scorer import _point_ranker, _sd
 
@@ -28,9 +27,10 @@ def test_point_scorer_activations(code, shape):
     s = r.forward(torch.from_numpy(z[key + "__X"]).to(DEV))
     assert rel_err(s.detach().cpu().numpy(), z[key + "__scores"]) <= 1e-5
     (s * torch.from_numpy(z[key + "__dscores"]).to(DEV)).sum().backward()
-    gscale = max(np.abs(z[f"{key}__grad::{k}"]).max() for k, _ in r.point_sf.named_parameters())
+    _, ref_grads = reference_point_outputs(z, key, F, AF=code, TL_AF=code, num_layers=3)
+    gscale = max(np.abs(g).max() for g in ref_grads.values())
     for k, p in r.point_sf.named_parameters():
-        ref = z[f"{key}__grad::{k}"]
+        ref = ref_grads[k]
         err = np.abs(p.grad.cpu().numpy() - ref).max()
         assert err <= 2e-5 * np.abs(ref).max() + 1e-6 * gscale + 1e-9, (k, err, np.abs(ref).max(), gscale)
 

@@ -4,8 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.helpers import load, rel_err
-from tests.test_oracle_vs_golden import POINT_CFGS, point_cfg
+from tests.helpers import POINT_CFGS, load, point_cfg, reference_point_outputs, rel_err
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -39,9 +38,10 @@ def test_point_scorer_forward_backward(name, shape):
     assert s.shape == (B, n)
     assert rel_err(s.detach().cpu().numpy(), z[key + "__scores"]) <= 1e-5
     (s * torch.from_numpy(z[key + "__dscores"]).to(DEV)).sum().backward()
-    gscale = max(np.abs(z[f"{key}__grad::{k}"]).max() for k, _ in r.point_sf.named_parameters())
+    _, ref_grads = reference_point_outputs(z, key, F, **POINT_CFGS[name])
+    gscale = max(np.abs(g).max() for g in ref_grads.values())
     for k, p in r.point_sf.named_parameters():
-        ref = z[f"{key}__grad::{k}"]
+        ref = ref_grads[k]
         err = np.abs(p.grad.cpu().numpy() - ref).max()
         # Linear biases feeding a norm have an exactly-zero true gradient: both sides hold pure rounding
         # noise there, hence the floor relative to the net's gradient scale

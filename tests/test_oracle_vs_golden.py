@@ -7,7 +7,7 @@ import torch
 
 from oracle import closed_form as cf
 from oracle import ref_port as rp
-from tests.helpers import load, loss_cases, parse_loss_key, rel_err
+from tests.helpers import POINT_CFGS, load, loss_cases, parse_loss_key, point_cfg, reference_point_outputs, rel_err  # noqa: F401
 
 CASES = loss_cases()
 
@@ -73,37 +73,14 @@ def _load_sd(z, prefix):
     return {k[len(prefix) + 2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith(prefix + "::")}
 
 
-POINT_CFGS = {
-    "default": dict(),
-    "bn2_relu": dict(AF="R", TL_AF="R", bn_type="BN2", bn_affine=False, num_layers=3),
-    "bn2_aff_celu": dict(AF="CE", TL_AF="S", bn_type="BN2", bn_affine=True, num_layers=2),
-    "nobn_sig_notl": dict(AF="S", TL_AF="S", BN=False, apply_tl_af=False, num_layers=4),
-    "bn_noaff_ge": dict(AF="GE", TL_AF="GE", bn_affine=False, num_layers=2),
-}
-
-
-def point_cfg(F, **over):
-    d = dict(num_features=F, num_layers=5, AF="GE", TL_AF="S", apply_tl_af=True,
-             BN=True, bn_type="BN", bn_affine=True, dropout=0.0)
-    d.update(over)
-    return d
-
-
 @pytest.mark.parametrize("name", list(POINT_CFGS))
 @pytest.mark.parametrize("shape", [(3, 50, 46), (2, 64, 136)])
 def test_point_scorer_port(name, shape):
     z = load("scorers.npz")
     B, n, F = shape
     key = f"point_{name}_B{B}_n{n}_F{F}"
-    net = rp.point_scorer(**point_cfg(F, **POINT_CFGS[name]))
-    net.load_state_dict(_load_sd(z, key + "__param"))
-    X = torch.from_numpy(z[key + "__X"])
-    s = rp.point_forward(net, X)
-    assert rel_err(s.detach().numpy(), z[key + "__scores"]) <= 2e-6
-    (s * torch.from_numpy(z[key + "__dscores"])).sum().backward()
-    for k, p in net.named_parameters():
-        ref = z[f"{key}__grad::{k}"]
-        assert np.abs(p.grad.numpy() - ref).max() <= 2e-5 * max(np.abs(ref).max(), 1e-3), k
+    s, _ = reference_point_outputs(z, key, F, **POINT_CFGS[name])      # checks every parameter gradient
+    assert rel_err(s, z[key + "__scores"]) <= 2e-6
 
 
 def list_sd_to_port(z, key):
