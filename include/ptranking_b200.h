@@ -136,6 +136,25 @@ int ptrb200_softrank_fwd_bwd(const float* scores, const float* labels, const int
 int ptrb200_sinkstep(const float* dist, const float* log_nu, const float* log_u, float* log_v,
                      int B, int d1, int d2, float lambda, ptrb200_stream_t stream);
 
+/* WassRank.custom_loss_function, mode 'SinkhornOT': ptranking/ltr_adhoc/listwise/wassrank/wassRank.py:43-86 with
+ * OldSinkhornOT (pytorch_wasserstein.py:323-394), the cost matrices of get_explicit_cost_mat and the histograms of
+ * get_normalized_histograms (wasserstein_cost_mat.py:47-244).  One CTA per query; the [n,n] cost matrix is rebuilt in
+ * registers from the labels and never stored.  The Sinkhorn updates run as row-wise log-sum-exps (finite in fp32 where
+ * the reference's per-vector stabilisation underflows).  loss_per_query[b] and the gradient carry 1/B_total (the
+ * reference's .mean(0) over the batch); B_total is the whole batch's query count, which a launch over one length bucket
+ * (B queries) needs passed in.  grad is the reference's envelope gradient (lam * log_u centred twice) chained through
+ * the histogram map.  gain_base, non_rele_gap, var_penalty: the 'eg' cost's parameters. */
+#define PTRB200_WASS_COST_EG   0   /* 'eg'  explicit grouping of the labels (torch_cost_mat_group) */
+#define PTRB200_WASS_COST_P1   1   /* 'p1'  |i - j| over positions */
+#define PTRB200_WASS_COST_P2   2   /* 'p2'  (i - j)^2 */
+#define PTRB200_WASS_COST_DG   3   /* 'dg'  |delta (2^y - 1)| */
+#define PTRB200_WASS_COST_DDG  4   /* 'ddg' |delta (2^y - 1)| * |delta 1/log2(rank + 2)| */
+#define PTRB200_WASS_SMOOTH_ST 0   /* 'ST' (norm_type 'BothST'): softmax of labels and of scores */
+#define PTRB200_WASS_SMOOTH_NG 1   /* 'NG': normalised gains 2^y - 1; scores over their sum, shifted by the min if <= 0 */
+int ptrb200_wassrank_fwd_bwd(const float* scores, const float* labels, const int32_t* offsets, float* grad, float* loss_per_query,
+                             int B, int n, int B_total, int cost_type, int smooth_type, float lam, int sh_itr,
+                             float gain_base, float non_rele_gap, float var_penalty, ptrb200_stream_t stream);
+
 /* deterministic (fixed-order) sum of n floats into out[0] -- the `torch.sum` over queries
  * that ends every reference loss (e.g. lambdarank.py:56). */
 int ptrb200_sum_f32(const float* x, float* out, int n, ptrb200_stream_t stream);

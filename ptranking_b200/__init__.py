@@ -17,10 +17,11 @@ from .ltr_adhoc.pointwise.rank_mse import RankMSE
 from .ltr_adhoc.listwise.rank_cosine import RankCosine
 from .ltr_adhoc.listwise.st_listnet import STListNet
 from .ltr_adhoc.listwise.softrank import SoftRank
+from .ltr_adhoc.listwise.wassrank import WassRank
 from .base.ranker import LABEL_TYPE
 
 MODELS = {c.__name__: c for c in (RankNet, LambdaRank, LambdaLoss, ListNet, ListMLE, ApproxNDCG,
-                                  RankMSE, RankCosine, STListNet, SoftRank)}
+                                  RankMSE, RankCosine, STListNet, SoftRank, WassRank)}
 __version__ = "0.1.0"
 
 

@@ -19,6 +19,8 @@ AF_CODES = {None: 0, "R": 1, "GE": 2, "S": 3, "T": 4, "CE": 5, "E": 6, "LR": 7, 
 NORM_CODES = {None: 0, "BN": 1, "BN2": 2}
 MATH_MODES = {"simt": 0, "3xtf32": 1, "tf32": 2, "bf16": 3}
 LAMBDALOSS_TYPES = {"NDCG_Loss1": 0, "NDCG_Loss2": 1, "NDCG_Loss2++": 2}
+WASS_COST_TYPES = {"eg": 0, "p1": 1, "p2": 2, "dg": 3, "ddg": 4}
+WASS_SMOOTH_TYPES = {"ST": 0, "NG": 1}
 
 _fp = C.c_void_p   # device pointers travel as integers
 
@@ -70,6 +72,7 @@ SIGNATURES = {
     "ptrb200_stlistnet_fwd_bwd": (_I, [_fp, _fp, _fp, _fp, _fp, _fp, _I, _I, _F, _U64, _U64, _fp]),
     "ptrb200_softrank_fwd_bwd": (_I, [_fp, _fp, _fp, _fp, _fp, _I, _I, _F, _I, _fp]),
     "ptrb200_sinkstep": (_I, [_fp, _fp, _fp, _fp, _I, _I, _I, _F, _fp]),
+    "ptrb200_wassrank_fwd_bwd": (_I, [_fp, _fp, _fp, _fp, _fp, _I, _I, _I, _I, _I, _F, _I, _F, _F, _F, _fp]),
     "ptrb200_standard_scale": (_I, [_fp, _fp, _fp, _I, _I, _I, _I, _F, _fp]),
     "ptrb200_sum_f32": (_I, [_fp, _fp, _I, _fp]),
     "ptrb200_ndcg_at_ks": (_I, [_fp, _fp, _fp, C.POINTER(C.c_int32), _I, _fp, _fp, _I, _I, _I, _fp]),

@@ -95,7 +95,7 @@ def _loss_call(name: str, scores: torch.Tensor, labels: torch.Tensor, params: di
     sp, gp, lq = s.data_ptr(), grad.data_ptr(), loss_q.data_ptr()
     # Length buckets pay for the O(n^2) losses only (the O(n) ones are launch-bound: one launch is best), and not for losses
     # coupled across the batch (ApproxNDCG's [B]/[B,1] broadcast, RankMSE's mean over queries)
-    quadratic = name in ("RankNet", "LambdaRank", "LambdaLoss", "SoftRank", "ApproxNDCG")
+    quadratic = name in ("RankNet", "LambdaRank", "LambdaLoss", "SoftRank", "ApproxNDCG", "WassRank")
     coupled = name == "RankMSE" or (name == "ApproxNDCG" and bool(params.get("batch_coupled", True)))
     ranges = _launch_ranges(B, n, offsets, params.get("buckets"), coupled or not quadratic)
     if name == "ListMLE":
@@ -124,6 +124,8 @@ def _loss_call(name: str, scores: torch.Tensor, labels: torch.Tensor, params: di
             seed = torch.initial_seed()
         if offset is None:
             offset = next_noise_offset()
+    if name == "WassRank":
+        wass = wassrank_settings(params)
     # ApproxNDCG scratch: Bq + 1 floats per launch; concurrent buckets get disjoint pieces
     scratch = torch.empty(B + len(ranges), dtype=torch.float32, device=s.device) if name == "ApproxNDCG" else None
     # The first bucket holds the longest lists: few CTAs that run long.  It goes onto a side stream so that the short-list
@@ -164,12 +166,36 @@ def _loss_call(name: str, scores: torch.Tensor, labels: torch.Tensor, params: di
         elif name == "SoftRank":
             top_k = params.get("top_k")
             rc = lib.ptrb200_softrank_fwd_bwd(sp, yp, opq, gp, lqq, Bq, nq, float(params.get("delta", 2.0)), int(top_k) if top_k else 0, st)
+        elif name == "WassRank":
+            rc = lib.ptrb200_wassrank_fwd_bwd(sp, yp, opq, gp, lqq, Bq, nq, B, *wass, st)
         else:
             raise NotImplementedError(name)
         _lib.check(rc, f"{name} loss kernel")
     if side is not None:
         torch.cuda.current_stream(s.device).wait_stream(side)
     return loss_q, grad
+
+
+def wassrank_settings(params: dict):
+    """WassRank's parameters (the keys of the reference's wass_para_dict, defaults of WassRankParameter,
+    wassRank.py:102-103) -> the kernel's (cost_type, smooth_type, lam, sh_itr, gain_base, non_rele_gap, var_penalty).
+    Raises NotImplementedError for what the reference does not run: mode 'EntropicOT' (not built here), any other mode,
+    smooth_type or norm_type, and unknown cost types (wassRank.py:79-80, wasserstein_cost_mat.py:136-137, :202-203, :243-244)."""
+    mode = params.get("mode", "SinkhornOT")
+    if mode == "EntropicOT":
+        raise NotImplementedError("WassRank mode 'EntropicOT' is not built in ptranking_b200; use mode='SinkhornOT'")
+    if mode != "SinkhornOT":
+        raise NotImplementedError(f"WassRank mode {mode!r}")
+    cost, smooth = params.get("cost_type", "eg"), params.get("smooth_type", "ST")
+    if cost not in _lib.WASS_COST_TYPES:
+        raise NotImplementedError(f"WassRank cost_type {cost!r}")
+    if smooth not in _lib.WASS_SMOOTH_TYPES:
+        raise NotImplementedError(f"WassRank smooth_type {smooth!r}")
+    if smooth == "ST" and params.get("norm_type", "BothST") != "BothST":
+        raise NotImplementedError(f"WassRank norm_type {params.get('norm_type')!r}")
+    return (_lib.WASS_COST_TYPES[cost], _lib.WASS_SMOOTH_TYPES[smooth], float(params.get("lam", 0.1)),
+            int(params.get("sh_itr", 20)), float(params.get("gain_base", 4)), float(params.get("non_rele_gap", 100)),
+            float(params.get("var_penalty", 2.718281828459045)))
 
 
 _side_streams = {}
